@@ -4,6 +4,7 @@ BASELINE.json's metric is quoted on, through libb200snark.so on 1..8 B200s; plus
 
   python bench.py --gpus N --steps K --warmup W            (torchrun for N > 1, one rank per GPU)
   python bench.py --impl reference ...                     (CPU restatement of the reference algorithms)
+  python bench.py ... --dump-outputs DIR                   (also write the last timed proof to DIR/proof_{a,b,c}.npy)
 
 One "step" = one proof: R1CS matrices x witness (SpMV) -> witness_map (the reference algorithm's 7 NTTs; 6 are executed, r1cs.cu) ->
 4 G1 MSMs + 1 G2 MSM -> epilogue.  Algorithmic bytes stay SURVEY 8(d)'s figure for the reference algorithm (7 transforms).
@@ -481,6 +482,8 @@ def run_b200(args):
             dist.destroy_process_group()
         return
     assert all(np.array_equal(x, y) for x, y in zip(proof_a, proof_b)), "resident and host-buffer proofs differ"
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, proof_a)
     verified = None
     if not args.no_verify:
         # regenerate every rank's key scalars on this GPU (same seeded generator) and check the proof in the exponent
@@ -534,6 +537,14 @@ def run_b200(args):
     emit(out)
     if world > 1:
         dist.destroy_process_group()
+
+
+def dump_outputs(path, proof):
+    """The proof of the last timed step as the caller receives it -- A (G1), B (G2), C (G1), affine, Montgomery u32 limbs --
+    one float64 array per point (exact for 32-bit words), so that two builds can be compared output for output."""
+    os.makedirs(path, exist_ok=True)
+    for name, arr in zip(("proof_a", "proof_b", "proof_c"), proof):
+        np.save(os.path.join(path, f"{name}.npy"), arr.astype(np.float64))
 
 
 def extras(be, torch, dev, ext, peak):
@@ -609,7 +620,12 @@ def main():
     ap.add_argument("--no-extras", action="store_true")
     ap.add_argument("--no-cpu", action="store_true")
     ap.add_argument("--no-verify", action="store_true", help="skip the one-off check of the proof against its known discrete logs")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the proof of the last timed step to DIR/proof_{a,b,c}.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs applies to the B200 arm")
     # the contract is ONE JSON line on stdout: anything libraries print there (e.g. NCCL's version banner) goes
     # to stderr instead; emit() writes the result line to the real stdout
     global _REAL_STDOUT
